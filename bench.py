@@ -58,7 +58,31 @@ def parse():
                     help="c2: BASELINE configs[1] + the metric's 80 lines (headline); c4: configs[3], chained align -> pose-opt at 720p")
     ap.add_argument("--sweep", action="store_true", help="BASELINE configs[4]: patch count x pyramid depth sweep (JSON list)")
     ap.add_argument("--sweep-out", default="", help="also write the sweep's JSON to this file (rank 0)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step of the device-resident leg returned as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "c4" or args.sweep):
+        ap.error("--dump-outputs is for the alignment leg (--config c2, --impl b200, no --sweep)")
+    return args
+
+
+DUMP_LIMIT = 64_000_000 - (1 << 16)  # bytes of array data: at most 64 MB written, with room left for the .npy headers
+DUMP_FIELDS = ("T_cur_w", "n_tracked", "H", "seg_killed", "iters", "status", "patch_iters", "patch_levels")
+
+
+def dump_outputs(out, directory):
+    """SparseImgAlign::run's outputs per pair as float64 .npy files (integer outputs are exact in float64).  A batch
+    whose outputs exceed DUMP_LIMIT is written as a fixed, seeded sample of pairs, listed in pair_index.npy."""
+    arrays = {n: np.asarray(getattr(out, n)).astype(np.float64) for n in DUMP_FIELDS}
+    B = len(arrays["T_cur_w"])
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    if B * row_bytes > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_LIMIT // (row_bytes + 8), replace=False))
+        arrays = {n: a[keep] for n, a in arrays.items()}
+        arrays["pair_index"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(directory, n + ".npy"), a)
 
 
 def workload_config(args, n_gpus):
@@ -672,6 +696,8 @@ def main():
     launches = ctx.launch_count() - launches0
     total_ms = float(sum(kernel_ms))
     out = al.download()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     t_total = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if dist:
         from plsvo_b200 import dist as pdist

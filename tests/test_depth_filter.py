@@ -8,38 +8,40 @@ whose last bit differs between glibc and the CUDA math library (tolerances state
 import numpy as np
 import pytest
 
+from reference_outputs import Reference
+
+SEED_FIELDS = ("status", "a", "b", "mu", "sigma2")
+
 
 @pytest.mark.parametrize("seed,kw", [(9000, {}), (9001, dict(n_pyr_levels=5)), (9002, dict(baseline=0.3)),
                                      (9003, dict(cam="QVGA")), (9004, dict(edgelet_frac=0.8))])
-def test_oracle_seed_update_is_bit_identical_to_the_reference_tus(oracle, abi, synth, seed, kw):
-    if not oracle.build_ref():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
+def test_oracle_seed_update_is_bit_identical_to_the_reference_tus(request, oracle, abi, synth, seed, kw):
+    oracle.build_ref()
     kw = dict(kw)
     if "cam" in kw:
         kw["cam"] = getattr(synth, kw["cam"])
     d = synth.make_seed_batch(n=1200, seed=seed, **kw)
     o = oracle.seed_update(abi, d, 4)
-    r = oracle.ref_seed_update(abi, d)
-    alive = r.status == 0  # the reference erases a seed whose variance reaches exactly 0 (converged): state not readable
+    r = Reference(request.node.name, d, lambda: oracle.ref_seed_update(abi, d), SEED_FIELDS)
+    alive = r.array("status") == 0  # the reference erases a seed whose variance reaches exactly 0 (converged): state not readable
     assert alive.mean() > 0.99
     for f in ("a", "b", "mu", "sigma2"):
-        np.testing.assert_array_equal(getattr(o, f)[alive], getattr(r, f)[alive], err_msg=f)
+        r.assert_equal(f, getattr(o, f)[alive], select=alive)
     assert set(np.unique(o.status)) == {0, 1, 2}
 
 
 @pytest.mark.parametrize("opts", [dict(align_1d=True), dict(subpix_refinement=False), dict(edgelet_filtering=False),
                                   dict(max_epi_search_steps=40)])
-def test_oracle_seed_update_matcher_options(oracle, abi, synth, opts):
-    if not oracle.build_ref():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
+def test_oracle_seed_update_matcher_options(request, oracle, abi, synth, opts):
+    oracle.build_ref()
     d = synth.make_seed_batch(n=800, seed=9010)
     for k, v in opts.items():
         setattr(d, k, v)
     o = oracle.seed_update(abi, d, 4)
-    r = oracle.ref_seed_update(abi, d)
-    alive = r.status == 0
+    r = Reference(request.node.name, d, lambda: oracle.ref_seed_update(abi, d), SEED_FIELDS)
+    alive = r.array("status") == 0
     for f in ("a", "b", "mu", "sigma2"):
-        np.testing.assert_array_equal(getattr(o, f)[alive], getattr(r, f)[alive], err_msg=f)
+        r.assert_equal(f, getattr(o, f)[alive], select=alive)
 
 
 def test_oracle_seed_update_measures_depth_and_shrinks_the_variance(oracle, abi, synth):
@@ -111,28 +113,27 @@ LINE_FIELDS = ("a", "b", "mu", "sigma2", "mu_e", "sigma2_e")
 
 
 @pytest.mark.parametrize("seed,kw", [(9500, {}), (9501, dict(n_pyr_levels=5)), (9502, dict(baseline=0.3)), (9503, dict(cam="QVGA"))])
-def test_oracle_line_seed_update_is_bit_identical_to_the_reference_tus(oracle, abi, synth, seed, kw):
-    if not oracle.build_ref():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
+def test_oracle_line_seed_update_is_bit_identical_to_the_reference_tus(request, oracle, abi, synth, seed, kw):
+    oracle.build_ref()
     kw = dict(kw)
     if "cam" in kw:
         kw["cam"] = getattr(synth, kw["cam"])
     d = synth.make_line_seed_batch(n=1000, seed=seed, **kw)
     o = oracle.line_seed_update(abi, d, 4)
-    r = oracle.ref_line_seed_update(abi, d)
-    alive = r.status == 0
+    r = Reference(request.node.name, d, lambda: oracle.ref_line_seed_update(abi, d), ("status",) + LINE_FIELDS)
+    alive = r.array("status") == 0
     assert alive.mean() > 0.99
     for f in LINE_FIELDS:
-        np.testing.assert_array_equal(getattr(o, f)[alive], getattr(r, f)[alive], err_msg=f)
+        r.assert_equal(f, getattr(o, f)[alive], select=alive)
     assert set(np.unique(o.status)) == {0, 1, 2}
     for opts in (dict(align_1d=True), dict(subpix_refinement=False), dict(max_epi_search_steps=30)):
         for k, v in opts.items():
             setattr(d, k, v)
         o = oracle.line_seed_update(abi, d, 4)
-        r = oracle.ref_line_seed_update(abi, d)
-        alive = r.status == 0
+        r = Reference(f"{request.node.name}/{opts}", d, lambda: oracle.ref_line_seed_update(abi, d), ("status",) + LINE_FIELDS)
+        alive = r.array("status") == 0
         for f in LINE_FIELDS:
-            np.testing.assert_array_equal(getattr(o, f)[alive], getattr(r, f)[alive], err_msg=f"{opts} {f}")
+            r.assert_equal(f, getattr(o, f)[alive], select=alive, err_msg=f"{opts} {f}")
 
 
 @pytest.mark.gpu

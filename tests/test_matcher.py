@@ -4,18 +4,18 @@ matcher.cpp compiled in place (oracle/_ref); the CUDA kernel must then be bit-id
 import numpy as np
 import pytest
 
+from reference_outputs import Reference
+
 
 @pytest.mark.parametrize("seed,levels,cam", [(7000, 3, "VGA"), (7001, 5, "VGA"), (7002, 3, "QVGA"), (7003, 4, "HD720")])
-def test_oracle_find_match_direct_is_bit_identical_to_the_reference_tu(oracle, abi, synth, seed, levels, cam):
-    if not oracle.build_ref():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
+def test_oracle_find_match_direct_is_bit_identical_to_the_reference_tu(request, oracle, abi, synth, seed, levels, cam):
+    oracle.build_ref()
     d = synth.make_match_batch(cam=getattr(synth, cam), n=1500, seed=seed, n_pyr_levels=levels)
     o = oracle.match_direct(abi, d, 4)
-    r = oracle.ref_match_direct(abi, d)
-    np.testing.assert_array_equal(o.success, r.success)
-    np.testing.assert_array_equal(o.search_level, r.search_level)
-    np.testing.assert_array_equal(o.px_cur, r.px_cur)
-    np.testing.assert_array_equal(o.A_cur_ref, r.A_cur_ref)  # Matcher::A_cur_ref_ (NaN = untouched on both sides)
+    fields = ("success", "search_level", "px_cur", "A_cur_ref")
+    r = Reference(request.node.name, d, lambda: oracle.ref_match_direct(abi, d), fields)
+    for f in fields:
+        r.assert_equal(f, getattr(o, f))  # A_cur_ref: Matcher::A_cur_ref_ (NaN = untouched on both sides)
     assert np.isfinite(o.A_cur_ref[o.search_level >= 0]).all()
     # the generator plants candidates on the image border: the in-frame test must reject them untouched
     assert (o.search_level < 0).any()

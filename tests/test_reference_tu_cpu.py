@@ -8,18 +8,19 @@ n_tracked, killed segments, per-level iteration counts, status; pose, covariance
 observation counts and outlier flags for the pose optimiser — over the edge cases the domain has
 (empty / ragged / masked feature lists, borders, zero motion, large motion, long segments, 720p).
 
-The library is built by __graft_entry__.build() / oracle_lib.build_ref() wherever /root/reference
-exists and travels as a prebuilt artefact otherwise; the tests skip only when neither is there.
+The library is built by __graft_entry__.build() / oracle_lib.build_ref() where the original sources are; elsewhere
+the tests compare with the record of its outputs (tests/reference_outputs.py).
 """
 import numpy as np
 import pytest
 
+from reference_outputs import Reference
+
 
 @pytest.fixture(scope="module")
 def ref(oracle, abi):
-    if not oracle.build_ref():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
-    oracle.load_ref(abi)
+    if oracle.build_ref():
+        oracle.load_ref(abi)
     return oracle
 
 
@@ -28,20 +29,19 @@ PO_FIELDS = ("T_f_w", "cov", "estimated_scale", "error_init", "error_final", "nu
              "seg_outlier", "status")
 
 
-def assert_align_identical(ref, abi, data, params=None, threads=4):
+def assert_align_identical(key, ref, abi, data, params=None, threads=4):
     a = ref.align(abi, data, params, n_threads=threads)
-    r = ref.ref_align(abi, data, params, n_threads=threads)
+    r = Reference(key, (data, params), lambda: ref.ref_align(abi, data, params, n_threads=threads), ALIGN_FIELDS)
     for f in ALIGN_FIELDS:
-        np.testing.assert_array_equal(getattr(a, f), getattr(r, f), err_msg=f)
+        r.assert_equal(f, getattr(a, f))
     return a
 
 
-def assert_poseopt_identical(ref, abi, data, params, rows=None):
+def assert_poseopt_identical(key, ref, abi, data, params):
     a = ref.poseopt(abi, data, params, n_threads=2)
-    r = ref.ref_poseopt(abi, data, params, n_threads=2)
-    rows = slice(None) if rows is None else rows
+    r = Reference(key, (data, params), lambda: ref.ref_poseopt(abi, data, params, n_threads=2), PO_FIELDS)
     for f in PO_FIELDS:
-        np.testing.assert_array_equal(getattr(a, f)[rows], getattr(r, f)[rows], err_msg=f)
+        r.assert_equal(f, getattr(a, f))
     return a
 
 
@@ -56,16 +56,16 @@ def assert_poseopt_identical(ref, abi, data, params, rows=None):
     dict(cam="HD720", batch=2, n_pts=500, n_segs=150, seed=109),                    # BASELINE config 4 shape
     dict(cam="QVGA", batch=6, n_pts=64, n_segs=16, seed=108, max_level=3, min_level=0),       # down to level 0
 ])
-def test_align_restatement_is_bit_identical_to_reference_tus(ref, abi, synth, cfg):
+def test_align_restatement_is_bit_identical_to_reference_tus(request, ref, abi, synth, cfg):
     cfg = dict(cfg)
     cfg["cam"] = getattr(synth, cfg["cam"])
     data = synth.make_align_batch(**cfg)
-    out = assert_align_identical(ref, abi, data)
+    out = assert_align_identical(request.node.name, ref, abi, data)
     if cfg["n_pts"]:
         assert (out.n_tracked > 0).all()
 
 
-def test_align_ragged_masked_and_empty_pairs(ref, abi, synth):
+def test_align_ragged_masked_and_empty_pairs(request, ref, abi, synth):
     data = synth.make_align_batch(cam=synth.QVGA, batch=12, n_pts=96, n_segs=40, seed=110)
     rng = np.random.default_rng(5)
     data.pt_valid = (rng.uniform(size=(12, 96)) > 0.2).astype(np.uint8)
@@ -78,20 +78,20 @@ def test_align_ragged_masked_and_empty_pairs(ref, abi, synth):
     data.seg_count[7] = 0  # points only
     data.pt_valid[9] = 0
     data.seg_valid[9] = 0  # features present but every feat3D == NULL
-    out = assert_align_identical(ref, abi, data)
+    out = assert_align_identical(request.node.name, ref, abi, data)
     assert out.status[3] & 1 and out.n_tracked[3] == 0
     np.testing.assert_array_equal(out.T_cur_w[3], data.T_cur_w[3])
 
 
-def test_align_zero_motion_raises_stop_like_the_reference(ref, abi, synth):
+def test_align_zero_motion_raises_stop_like_the_reference(request, ref, abi, synth):
     """cur == ref: every residual is 0, the per-segment mean residual is 0 and H_*weight/res_ divides by it
     (sparse_img_align.cpp:676): the solve returns NaN and vk::NLLSSolver raises stop_."""
     data = synth.make_align_batch(cam=synth.QVGA, batch=3, n_pts=64, n_segs=16, seed=111, motion_t=0.0, motion_r=0.0)
-    out = assert_align_identical(ref, abi, data)
+    out = assert_align_identical(request.node.name, ref, abi, data)
     assert (out.status & 2).all()
 
 
-def test_align_long_segments_and_iteration_limits(ref, abi, synth):
+def test_align_long_segments_and_iteration_limits(request, ref, abi, synth):
     """Segments spanning the image (many 4x4 samples each, some samples leaving the frame -> killed segments),
     at levels 2..0, and tight iteration / level limits."""
     import torch
@@ -115,9 +115,10 @@ def test_align_long_segments_and_iteration_limits(ref, abi, synth):
     data.seg_sf, data.seg_spos = (np.ascontiguousarray(x) for x in lift(spx))
     data.seg_ef, data.seg_epos = (np.ascontiguousarray(x) for x in lift(epx))
     data.seg_length = np.ascontiguousarray(np.linalg.norm(epx - spx, axis=-1))
-    assert_align_identical(ref, abi, data, abi.align_params(2, 0, 30))
-    assert_align_identical(ref, abi, data, abi.align_params(2, 1, 3))   # n_iter = 3
-    assert_align_identical(ref, abi, data, abi.align_params(2, 2, 30))  # a single level
+    key = request.node.name
+    assert_align_identical(key + "/2-0", ref, abi, data, abi.align_params(2, 0, 30))
+    assert_align_identical(key + "/2-1", ref, abi, data, abi.align_params(2, 1, 3))   # n_iter = 3
+    assert_align_identical(key + "/2-2", ref, abi, data, abi.align_params(2, 2, 30))  # a single level
 
 
 @pytest.mark.parametrize("n_ref", [-1, 0, 5])
@@ -128,12 +129,12 @@ def test_align_long_segments_and_iteration_limits(ref, abi, synth):
     dict(batch=12, seed=204, noise_px=2.0, pert_t=0.08, pert_r=0.04),
     dict(batch=12, seed=205, noise_px=0.0, outlier_frac=0.0),
 ])
-def test_poseopt_restatement_is_bit_identical_to_reference_tus(ref, abi, synth, cfg, n_ref):
+def test_poseopt_restatement_is_bit_identical_to_reference_tus(request, ref, abi, synth, cfg, n_ref):
     data = synth.make_poseopt_batch(**cfg)
-    assert_poseopt_identical(ref, abi, data, abi.poseopt_params(2.0, 10, n_ref))
+    assert_poseopt_identical(request.node.name, ref, abi, data, abi.poseopt_params(2.0, 10, n_ref))
 
 
-def test_poseopt_ragged_and_masked(ref, abi, synth):
+def test_poseopt_ragged_and_masked(request, ref, abi, synth):
     data = synth.make_poseopt_batch(batch=10, n_pts=64, n_segs=24, seed=210)
     rng = np.random.default_rng(9)
     data.pt_valid = (rng.uniform(size=(10, 64)) > 0.25).astype(np.uint8)
@@ -143,27 +144,31 @@ def test_poseopt_ragged_and_masked(ref, abi, synth):
     data.pt_valid[2] = 0
     data.seg_valid[2] = 0  # no observations at all: early return (pose_optimizer.cpp:88-89)
     for n_ref in (-1, 4):
-        out = assert_poseopt_identical(ref, abi, data, abi.poseopt_params(2.0, 10, n_ref))
+        out = assert_poseopt_identical(f"{request.node.name}/{n_ref}", ref, abi, data, abi.poseopt_params(2.0, 10, n_ref))
         assert out.status[2] == 1
         np.testing.assert_array_equal(out.T_f_w[2], data.T_f_w[2])
 
 
-def test_golden_fixtures_are_reference_outputs(ref, abi, synth):
-    """tests/golden/*.npz were written from oracle/_ref (tests/golden/make_golden.py): regenerating them here
-    must give the same bits, i.e. the committed vectors ARE what the reference's own code computes."""
+def test_golden_fixtures_are_reference_outputs(request, ref, abi, synth):
+    """tests/golden/*.npz were written from oracle/_ref (tests/golden/make_golden.py): what the reference's own code
+    computes on their inputs must be the committed vectors bit for bit."""
     from golden_io import load_align, load_poseopt
 
     d, z = load_align(synth)
-    r = ref.ref_align(abi, d, abi.align_params(3, 1, 30))
+    p = abi.align_params(3, 1, 30)
+    fields = ("T_cur_w", "n_tracked", "H", "seg_killed", "iters")
+    r = Reference(request.node.name + "/align", (d, p), lambda: ref.ref_align(abi, d, p), fields)
     assert "sparse_img_align" in str(z["source"])
-    for f in ("T_cur_w", "n_tracked", "H", "seg_killed", "iters"):
-        np.testing.assert_array_equal(getattr(r, f), z[f"out_{f}"], err_msg=f)
+    for f in fields:
+        r.assert_equal(f, z[f"out_{f}"])
     d, z = load_poseopt(synth)
+    fields = ("T_f_w", "cov", "estimated_scale", "error_init", "error_final", "num_obs_pt", "num_obs_ls", "pt_outlier",
+              "seg_outlier")
     for tag, n_ref in (("9arg", -1), ("10arg", 3)):
-        r = ref.ref_poseopt(abi, d, abi.poseopt_params(2.0, 10, n_ref))
-        for f in ("T_f_w", "cov", "estimated_scale", "error_init", "error_final", "num_obs_pt", "num_obs_ls", "pt_outlier",
-                  "seg_outlier"):
-            np.testing.assert_array_equal(getattr(r, f), z[f"out_{tag}_{f}"], err_msg=f"{tag} {f}")
+        p = abi.poseopt_params(2.0, 10, n_ref)
+        r = Reference(f"{request.node.name}/{tag}", (d, p), lambda: ref.ref_poseopt(abi, d, p), fields)
+        for f in fields:
+            r.assert_equal(f, z[f"out_{tag}_{f}"], err_msg=f"{tag} {f}")
 
 
 def test_shim_packs_reference_objects_like_the_reference_reads_them(ref, abi, synth):
@@ -197,13 +202,13 @@ def test_shim_packs_reference_objects_like_the_reference_reads_them(ref, abi, sy
             np.testing.assert_allclose(getattr(got, f), getattr(want, f), rtol=1e-12, err_msg=f)
 
 
-def test_sequence_chain_oracle_equals_reference_chain(abi, synth, oracle):
+def test_sequence_chain_oracle_equals_reference_chain(request, abi, synth, oracle):
     """BASELINE config 1 on the CPU: frame-to-frame chain (align -> pose-opt, the estimate seeds the next frame,
     frame_handler_mono.cpp:263-340) over short QVGA sequences — the oracle restatement and the reference's own
     translation units give bit-identical poses, iteration counts and outlier flags at every frame, and the chain tracks
     the ground-truth trajectory."""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
+    if oracle.build_ref():
+        oracle.load_ref(abi)
     poses, steps = synth.make_sequence(cam=synth.QVGA, n_seq=2, n_frames=6, n_pts=120, n_segs=30, seed=1000)
 
     def chain(align_fn, po_fn):
@@ -213,10 +218,11 @@ def test_sequence_chain_oracle_equals_reference_chain(abi, synth, oracle):
             return ra, po_fn(abi, po, abi.poseopt_params(2.0, 10, -1), n_threads=4)
         return synth.run_sequence(poses, steps, step)
 
+    r = Reference(request.node.name, (poses, steps),
+                  lambda: dict(zip(("est", "iters", "outliers"), chain(oracle.ref_align, oracle.ref_poseopt))))
     est_o, it_o, out_o = chain(oracle.align, oracle.poseopt)
-    est_r, it_r, out_r = chain(oracle.ref_align, oracle.ref_poseopt)
-    np.testing.assert_array_equal(est_o, est_r)
-    np.testing.assert_array_equal(it_o, it_r)
-    np.testing.assert_array_equal(out_o, out_r)
-    ang, rel = synth.pose_error(est_r[:, -1], poses[:, -1])
+    r.assert_equal("est", est_o)
+    r.assert_equal("iters", it_o)
+    r.assert_equal("outliers", out_o)
+    ang, rel = synth.pose_error(est_o[:, -1], poses[:, -1])
     assert ang.max() < 1e-2

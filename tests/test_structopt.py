@@ -4,18 +4,19 @@ The oracle restatement is pinned bit for bit against the reference's own feature
 import numpy as np
 import pytest
 
+from reference_outputs import Reference
+
 
 @pytest.mark.parametrize("seed,n_iter", [(8000, 5), (8001, 20), (8002, 1), (8003, 0)])
-def test_oracle_structopt_is_bit_identical_to_the_reference_tu(oracle, abi, synth, seed, n_iter):
-    if not oracle.build_ref():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
+def test_oracle_structopt_is_bit_identical_to_the_reference_tu(request, oracle, abi, synth, seed, n_iter):
+    oracle.build_ref()
     d = synth.make_structopt_batch(n_points=1200, n_segs=300, seed=seed)
     d.n_iter_pts = d.n_iter_segs = n_iter
     o = oracle.structopt(abi, d, 4)
-    r = oracle.ref_structopt(abi, d)
-    np.testing.assert_array_equal(o.pt_pos, r.pt_pos)
-    np.testing.assert_array_equal(o.seg_spos, r.seg_spos)
-    np.testing.assert_array_equal(o.seg_epos, r.seg_epos)
+    fields = ("pt_pos", "seg_spos", "seg_epos")
+    r = Reference(request.node.name, d, lambda: oracle.ref_structopt(abi, d), fields)
+    for f in fields:
+        r.assert_equal(f, getattr(o, f))
     if n_iter == 0:
         np.testing.assert_array_equal(o.pt_pos, d.pt_pos)
 
