@@ -56,7 +56,8 @@ struct PairCtl {
   double x[6];
   unsigned long long mbar;
   long long n_meas_last;
-  int pair;
+  int pair;      // work-queue ticket of the current unit
+  int level_lo;  // finest level of the current unit
   int flag;
   int stop;
   int iter;
@@ -518,6 +519,39 @@ __device__ __forceinline__ uint2 make_item(uint32_t Ae, uint32_t Ao, uint32_t ef
   return it;
 }
 
+// ---- level units: a pair's progress word and the state it carries between levels (global memory, L2) ----
+__device__ __forceinline__ unsigned long long ld_acquire_gpu(const unsigned long long* p) {
+  unsigned long long v;
+  asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void st_release_gpu(unsigned long long* p, unsigned long long v) {
+  asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __noinline__ void unit_state_store(const PairCtl* ctl, AlignUnitState* s) {
+  for (int i = 0; i < 7; ++i) s->model[i] = ctl->model[i];
+  for (int i = 0; i < 9; ++i) s->R[i] = ctl->R[i];
+  for (int i = 0; i < 3; ++i) s->t[i] = ctl->t[i];
+  s->chi2_prev = ctl->chi2_prev;
+  for (int i = 0; i < 36; ++i) s->H_last[i] = ctl->H_last[i];
+  s->n_meas_last = ctl->n_meas_last;
+  s->stop = ctl->stop, s->chi2_flags = ctl->chi2_flags;
+  s->patch_iters = ctl->patch_iters, s->patch_levels = ctl->patch_levels;
+  for (int l = 0; l < PLSVO_MAX_LEVELS; ++l) s->iters_level[l] = ctl->iters_level[l];
+}
+// L2 loads (ld.global.cg): the state was written by another SM
+__device__ __noinline__ void unit_state_load(PairCtl* ctl, const AlignUnitState* s) {
+  for (int i = 0; i < 7; ++i) ctl->model[i] = __ldcg(s->model + i);
+  for (int i = 0; i < 9; ++i) ctl->R[i] = __ldcg(s->R + i);
+  for (int i = 0; i < 3; ++i) ctl->t[i] = __ldcg(s->t + i);
+  ctl->chi2_prev = __ldcg(&s->chi2_prev);
+  for (int i = 0; i < 36; ++i) ctl->H_last[i] = __ldcg(s->H_last + i);
+  ctl->n_meas_last = __ldcg(&s->n_meas_last);
+  ctl->stop = __ldcg(&s->stop), ctl->chi2_flags = __ldcg(&s->chi2_flags);
+  ctl->patch_iters = __ldcg(&s->patch_iters), ctl->patch_levels = __ldcg(&s->patch_levels);
+  for (int l = 0; l < PLSVO_MAX_LEVELS; ++l) ctl->iters_level[l] = __ldcg(s->iters_level + l);
+}
+
 template <int NT, int MINB>
 __global__ void __launch_bounds__(NT, MINB) sparse_img_align_kernel(const AlignArgs a) {
   constexpr int NW = NT / 32;
@@ -562,7 +596,8 @@ __global__ void __launch_bounds__(NT, MINB) sparse_img_align_kernel(const AlignA
   }
   __syncthreads();
   uint32_t bar_parity = 0;
-
+  // Work queue.  Pair mode: ticket = pair.  Level units: ticket = (level index k, pair), k-major, so the unit of pair b at
+  // level max_level - k is ticket k*B + b and the unit it continues from was handed out exactly B tickets earlier.
   for (;;) {
     __syncthreads();  // everyone is done with ctl of the previous pair
     if (tid == 0) {
@@ -575,10 +610,13 @@ __global__ void __launch_bounds__(NT, MINB) sparse_img_align_kernel(const AlignA
         __threadfence_system();
       }
       ctl->pair = nb;
+      ctl->level_lo = a.level_units ? a.max_level - nb / a.B : a.min_level;
     }
     __syncthreads();
-    const int b = ctl->pair;
-    if (b >= a.B) break;
+    const int ticket = ctl->pair;
+    if (ticket >= a.B * (a.level_units ? a.max_level - a.min_level + 1 : 1)) break;
+    const int unit = ticket / a.B;  // levels of this pair done before this unit
+    const int b = ticket - unit * a.B;
 
     // feature counts are validated on upload; the clamp keeps a corrupted count from indexing out of bounds
     const int np = min(max(a.pt_count ? a.pt_count[b] : a.n_pts, 0), a.n_pts);
@@ -586,6 +624,7 @@ __global__ void __launch_bounds__(NT, MINB) sparse_img_align_kernel(const AlignA
     const size_t po = (size_t)b * a.n_pts, so = (size_t)b * a.n_segs;
 
     if (np == 0 && ns == 0) {  // :58-62 early-out: return 0, cur pose untouched
+      if (unit > 0) continue;  // the pair's first unit has written its outputs; nobody waits for an empty pair
       if (tid == 0) {
         for (int i = 0; i < 7; ++i) a.out_T[(size_t)b * 7 + i] = a.T_cur_w[(size_t)b * 7 + i];
         a.out_n_tracked[b] = 0;
@@ -601,23 +640,25 @@ __global__ void __launch_bounds__(NT, MINB) sparse_img_align_kernel(const AlignA
 
     if (tid == 0) {
       const SE3q T_ref = se3_load(a.T_ref_w + (size_t)b * 7);
-      const SE3q T_cur = se3_load(a.T_cur_w + (size_t)b * 7);
       const SE3q T_ref_inv = se3_inverse(T_ref);
-      const SE3q model = se3_mul(T_cur, T_ref_inv);  // :80
       se3_store(T_ref, ctl->T_ref);
-      se3_store(model, ctl->model);
       ctl->ref_pos[0] = T_ref_inv.t.x, ctl->ref_pos[1] = T_ref_inv.t.y, ctl->ref_pos[2] = T_ref_inv.t.z;
-      quat_to_R(model.q, ctl->R);
-      ctl->t[0] = model.t.x, ctl->t[1] = model.t.y, ctl->t[2] = model.t.z;
-      ctl->chi2_prev = 1e10;
-      ctl->stop = 0;
-      ctl->n_meas_last = 0;
-      ctl->patch_iters = 0;
-      ctl->patch_levels = 0;
-      ctl->chi2_flags = 0;
       ctl->n_opq = 0;
-      for (int i = 0; i < 36; ++i) ctl->H_last[i] = 0.0;
-      for (int l = 0; l < PLSVO_MAX_LEVELS; ++l) ctl->iters_level[l] = 0;
+      if (unit == 0) {
+        const SE3q T_cur = se3_load(a.T_cur_w + (size_t)b * 7);
+        const SE3q model = se3_mul(T_cur, T_ref_inv);  // :80
+        se3_store(model, ctl->model);
+        quat_to_R(model.q, ctl->R);
+        ctl->t[0] = model.t.x, ctl->t[1] = model.t.y, ctl->t[2] = model.t.z;
+        ctl->chi2_prev = 1e10;
+        ctl->stop = 0;
+        ctl->n_meas_last = 0;
+        ctl->patch_iters = 0;
+        ctl->patch_levels = 0;
+        ctl->chi2_flags = 0;
+        for (int i = 0; i < 36; ++i) ctl->H_last[i] = 0.0;
+        for (int l = 0; l < PLSVO_MAX_LEVELS; ++l) ctl->iters_level[l] = 0;
+      }
     }
     // Host-buffer pipeline with lean inputs: pyramid levels above a.derive_from were not shipped; this CTA forms them
     // for its own pair by vk::halfSample (truncating 2x2 mean, frame_utils::createImgPyramid, src/frame.cpp:171-180)
@@ -669,11 +710,25 @@ __global__ void __launch_bounds__(NT, MINB) sparse_img_align_kernel(const AlignA
       seg_alive[j] = a.seg_valid ? (a.seg_valid[so + j] ? 1 : 0) : 1;
       seg_N0[j] = seg_num_samples0(a.seg_spx + (so + j) * 2, a.seg_epx + (so + j) * 2, a.seg_length[so + j]);
     }
+    if (unit > 0) {
+      const unsigned char* ust = a.unit_state + (size_t)b * a.unit_state_stride;
+      // Continue the pair where the unit of the level above left it.  No deadlock: that unit holds ticket - B, which was
+      // handed out before this one, so a resident CTA is running it; and it only ever waits for a ticket earlier still.
+      if (tid == 0) {
+        const unsigned long long want = (a.unit_epoch << 4) | (unsigned long long)unit;
+        while (ld_acquire_gpu(a.unit_done + b) != want) __nanosleep(256);
+        unit_state_load(ctl, reinterpret_cast<const AlignUnitState*>(ust));
+      }
+      __syncthreads();
+      const unsigned char* vis = ust + sizeof(AlignUnitState);
+      for (int i = tid; i < np; i += NT) pt_vis[i] = __ldcg(vis + i);
+      for (int j = tid; j < ns; j += NT) seg_alive[j] = __ldcg(vis + a.n_pts + j);
+    }
     unsigned int my_patch_levels = 0;
     const int n_chunks = (np + 31) >> 5;       // 32-patch chunks of the point list
     const int rounds = (np + NT - 1) / NT;     // rounds of NT point patches per pass
 
-    for (int level = a.max_level; level >= a.min_level; --level) {
+    for (int level = a.level_units ? ctl->level_lo : a.max_level; level >= ctl->level_lo; --level) {
       const int cols = a.width >> level, rows = a.height >> level;
       const int pitch = (int)a.pitch[level];
       const float scale = 1.0f / (float)(1 << level);
@@ -1190,6 +1245,19 @@ __global__ void __launch_bounds__(NT, MINB) sparse_img_align_kernel(const AlignA
 #pragma unroll
       for (int d = 16; d >= 1; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
       if (lane == 0 && v) atomicAdd(&ctl->patch_levels, v);
+    }
+    if (ctl->level_lo > a.min_level) {  // hand the pair on to its unit at the next finer level
+      unsigned char* ust = a.unit_state + (size_t)b * a.unit_state_stride;
+      unsigned char* vis = ust + sizeof(AlignUnitState);
+      for (int i = tid; i < np; i += NT) vis[i] = pt_vis[i];
+      for (int j = tid; j < ns; j += NT) vis[a.n_pts + j] = seg_alive[j];
+      __syncthreads();
+      if (tid == 0) {
+        unit_state_store(ctl, reinterpret_cast<AlignUnitState*>(ust));
+        __threadfence();
+        st_release_gpu(a.unit_done + b, (a.unit_epoch << 4) | (unsigned long long)(a.max_level - ctl->level_lo + 1));
+      }
+      continue;
     }
     for (int j = tid; j < a.n_segs; j += NT) {
       const bool valid0 = (j < ns) && (a.seg_valid ? a.seg_valid[so + j] != 0 : true);

@@ -66,7 +66,29 @@ struct AlignArgs {
   int rec_cap;          // 32-sample trips of the longest segment, <= 32
   int derive_from;      // >= 0: the CTA forms levels (derive_from, max_level] of its pair by halfSample (gated pipeline)
   float one;            // 1.0f, deliberately a run-time value (device_math.cuh: add2_after_mul)
+  // level units (DESIGN.md §4.1): the work queue hands out (pair, level) tickets, level-major, instead of whole pairs.
+  // A pair's state between two levels goes through unit_state; unit_done[b] = (unit_epoch << 4) | levels of pair b done.
+  int level_units;
+  unsigned long long unit_epoch;  // counts the launches of the context from 1 (the words are cleared to 0 when allocated)
+  unsigned long long* unit_done;  // [B]
+  unsigned char* unit_state;     // [B][unit_state_stride]: AlignUnitState, pt_vis[n_pts], seg_alive[n_segs]
+  size_t unit_state_stride;
 };
+
+// What a pair carries from one Gauss-Newton level to the next; everything else is rebuilt at the start of a level or
+// recomputed from the inputs with identical bits.
+struct AlignUnitState {
+  double model[7], R[9], t[3];
+  double chi2_prev;
+  double H_last[36];
+  long long n_meas_last;
+  int stop, chi2_flags;
+  unsigned int patch_iters, patch_levels;
+  int iters_level[PLSVO_MAX_LEVELS];
+};
+inline size_t align_unit_state_stride(int n_pts, int n_segs) {
+  return (sizeof(AlignUnitState) + (size_t)n_pts + (size_t)n_segs + 127) / 128 * 128;
+}
 
 // shared memory the kernel needs for a configuration (host + device agree through this)
 size_t align_smem_bytes(int n_pts, int n_segs, int max_patches, int max_seg_slots, int img_bytes, int threads);

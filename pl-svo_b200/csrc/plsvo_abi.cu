@@ -70,6 +70,8 @@ struct plsvo_ctx_impl {
       d_seg_spx, d_seg_epx, d_seg_sf, d_seg_ef, d_seg_spos, d_seg_epos, d_seg_length, d_seg_valid;
   DevBuf d_out_T, d_out_ntr, d_out_H, d_out_killed, d_out_iters, d_out_status, d_out_pi, d_out_pl, d_counter,
       d_ws_cache, d_ws_xyz, d_ws_segpx, d_ws_rec, d_stage;
+  DevBuf d_unit_done, d_unit_state;  // level units: per-pair progress words and the state carried between levels
+  unsigned long long unit_epoch = 0;
   size_t level_off[PLSVO_MAX_LEVELS];
 
   // ---- pose-opt state ----
@@ -223,7 +225,7 @@ void plsvo_ctx_destroy(plsvo_ctx* ctx) {
                     &c->d_pt_f,      &c->d_pt_pos,   &c->d_pt_valid,  &c->d_seg_count,  &c->d_seg_spx,   &c->d_seg_epx,
                     &c->d_seg_sf,    &c->d_seg_ef,   &c->d_seg_spos,  &c->d_seg_epos,   &c->d_seg_length, &c->d_seg_valid,
                     &c->d_out_T,     &c->d_out_ntr,  &c->d_out_H,     &c->d_out_killed, &c->d_out_iters, &c->d_out_status,
-                    &c->d_out_pi,    &c->d_out_pl,   &c->d_counter,   &c->d_ws_cache,   &c->d_ws_xyz,    &c->d_ref_der,   &c->d_cur_der,   &c->d_pt_depth,  &c->d_seg_sdepth, &c->d_seg_edepth, &c->d_feat, &c->d_ws_segpx,  &c->d_ws_rec,    &c->d_stage,     &c->y_img,       &c->f_img,       &c->f_idx,       &c->f_lvl,      &c->f_border,
+                    &c->d_out_pi,    &c->d_out_pl,   &c->d_counter,   &c->d_ws_cache,   &c->d_ws_xyz,    &c->d_ref_der,   &c->d_cur_der,   &c->d_pt_depth,  &c->d_seg_sdepth, &c->d_seg_edepth, &c->d_feat, &c->d_ws_segpx,  &c->d_ws_rec,    &c->d_stage,     &c->d_unit_done, &c->d_unit_state, &c->y_img,       &c->f_img,       &c->f_idx,       &c->f_lvl,      &c->f_border,
                     &c->f_ref,       &c->f_px,        &c->f_opx,       &c->f_oconv,     &c->f_dir,       &c->f_ohinv,     &c->m_ref_img,   &c->m_cur_img,   &c->m_T_ref,     &c->m_T_cur,
                     &c->m_ridx,      &c->m_cidx,     &c->m_px,        &c->m_f,          &c->m_lvl,       &c->m_edge,
                     &c->m_grad,      &c->m_pos,      &c->m_pxc,       &c->m_opx,        &c->m_osucc,     &c->m_olvl,      &c->m_oA,        &c->s_T,         &c->s_pb,        &c->s_pf,        &c->s_pof,
@@ -883,9 +885,10 @@ int align_plan(plsvo_ctx_impl* c, const plsvo_align_params* p, int chunk_pairs, 
   return rc_last;
 }
 
-// one kernel over pairs [b0,b1) of the uploaded batch (pointers rebased to the chunk)
+// one kernel over pairs [b0,b1) of the uploaded batch (pointers rebased to the chunk).  units_ok: the whole batch in one
+// ungated launch, where the work queue may hand out (pair, level) units (see below).
 int align_launch_range(plsvo_ctx_impl* c, const AlignPlan& plan, size_t b0, size_t b1, int counter_slot, cudaStream_t s,
-                       int gate_chunk = 0) {
+                       int gate_chunk = 0, bool units_ok = false) {
   AlignArgs a = c->aa;
   const size_t np = (size_t)a.n_pts, ns = (size_t)a.n_segs;
   a.B = (int)(b1 - b0);
@@ -927,7 +930,31 @@ int align_launch_range(plsvo_ctx_impl* c, const AlignPlan& plan, size_t b0, size
   a.work_counter = c->aa.work_counter + counter_slot;
   a.arrived = gate_chunk > 0 ? c->aa.work_counter + 32 : nullptr;
   a.gate_chunk = gate_chunk;
-  const int grid = std::min(a.B, c->num_sms * plan.ctas_per_sm);
+  const int slots = c->num_sms * plan.ctas_per_sm;
+  const int grid = std::min(a.B, slots);
+  // Level units: a persistent slot that owns a whole pair idles once the queue is empty while the slowest pairs of the
+  // second wave finish.  When the batch has more pairs than the grid has slots, the queue hands out (pair, level) units
+  // instead — same CTA shape, same arithmetic, bit-identical results — so the ragged end shrinks to a fraction of a pair.
+  // Not on the arrival-gated path (pairs trickle in) nor with levels the kernel derives itself.
+  // PLSVO_ALIGN_SCHEDULE=pair|level forces either mode (A/B runs, tests).
+  bool units = units_ok && gate_chunk == 0 && a.derive_from < 0 && a.max_level > a.min_level && a.B > slots;
+  if (const char* e = getenv("PLSVO_ALIGN_SCHEDULE")) {
+    if (!strcmp(e, "pair")) units = false;
+    else if (!strcmp(e, "level")) units = units_ok && gate_chunk == 0 && a.derive_from < 0;
+  }
+  a.level_units = units ? 1 : 0;
+  if (units) {
+    const size_t done_bytes = (size_t)a.B * sizeof(unsigned long long);
+    if (c->d_unit_done.cap < done_bytes) {  // fresh words must not match any epoch
+      CK(ensure(c->d_unit_done, done_bytes));
+      CK(cudaMemsetAsync(c->d_unit_done.p, 0, c->d_unit_done.cap, s));
+    }
+    a.unit_state_stride = align_unit_state_stride(a.n_pts, a.n_segs);
+    CK(ensure(c->d_unit_state, (size_t)a.B * a.unit_state_stride));
+    a.unit_done = static_cast<unsigned long long*>(c->d_unit_done.p);
+    a.unit_state = static_cast<unsigned char*>(c->d_unit_state.p);
+    a.unit_epoch = ++c->unit_epoch;
+  }
   CK(cudaMemsetAsync(a.work_counter, 0, sizeof(unsigned int), s));
   CK(align_kernel_launch(a, grid, plan.threads, plan.min_blocks, plan.smem, s));
   c->launches += 1;
@@ -955,7 +982,7 @@ int plsvo_align_launch(plsvo_ctx* ctx, const plsvo_align_params* p) {
   if (rc != PLSVO_OK) return rc;
   rc = align_plan(c, p, c->aa.B, &plan);
   if (rc != PLSVO_OK) return rc;
-  return align_launch_range(c, plan, 0, (size_t)c->aa.B, 0, c->stream);
+  return align_launch_range(c, plan, 0, (size_t)c->aa.B, 0, c->stream, 0, /*units_ok=*/true);
 }
 
 int plsvo_align_download(plsvo_ctx* ctx, const plsvo_align_result* o) {
